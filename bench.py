@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...   # the CPU restatement on the host cores
+    python bench.py ... --dump-outputs DIR                   # also save the last timed step's outputs (seeded inputs)
 
 A "step" is one pass of the hot path over one batch: ONE Gym env-step (frame_skip = 10 physics
 substeps, obs, reward, termination, auto-reset) of every environment of the batch. At N = 1 the
@@ -292,11 +293,15 @@ def run_gpu(args):
     for i in range(K):
         flush.zero_()                                # evict L2 between timed steps (not timed)
         starts[i].record()
-        env.step(actions[W + i])
+        out = env.step(actions[W + i])
         ends[i].record()
     barrier()
     wall = time.perf_counter() - t_wall0
     launches = env.launch_count - launches0
+    if args.dump_outputs:
+        # copied now: obs and reward are views of the env's output buffer, which the e2e steps below overwrite
+        obs, rew, done, _ = out
+        dump_outputs(args.dump_outputs, {"obs": obs, "reward": rew, "done": done}, rank, world)
     dev_ms = sum(s.elapsed_time(e) for s, e in zip(starts, ends))
     # ---- e2e: host buffers in, host results out, every step
     h_act = torch.empty(N, 8, pin_memory=True)
@@ -412,6 +417,29 @@ def run_gpu(args):
     if dist is not None:
         dist.destroy_process_group()
     return 0
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, rank, world):
+    """Write what the last timed step returned as `<name>.npy` in float32 (`<name>.rank<r>.npy` with several ranks), so
+    that two builds can be compared output for output. Above DUMP_MAX_BYTES a fixed, seeded sample of environments is
+    written, with their indices in `env_index.npy`."""
+    import numpy as np
+    import torch
+    arrays = {k: v.detach().to("cpu", torch.float32).numpy() for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a.nbytes for a in arrays.values()) // n
+    budget = DUMP_MAX_BYTES - 4096                   # room for the .npy headers
+    if n * row_bytes > budget:
+        idx = np.sort(np.random.default_rng(0).choice(n, budget // (row_bytes + 8), replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["env_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = f".rank{rank}" if world > 1 else ""
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}{suffix}.npy"), a)
 
 
 def large_batch_probe(dev, n_envs, extra=None, model="our_robot"):
@@ -614,7 +642,10 @@ def main():
     ap.add_argument("--mppi", type=int, default=1, help="N=1: also time one MPPI plan (1024 x 64); 0 = off")
     ap.add_argument("--train-probe", action="store_true", help="N=1: include the PPO epoch in the rollout probe")
     ap.add_argument("--cfg", action="append", default=[], help="OdgEnvConfig override key=value (experiments)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's obs / reward / done to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     return run_gpu(args)

@@ -8,25 +8,20 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_XML = "/root/reference/Code/mujoco/our_robot/walking_scene.xml"
 
 
-@pytest.mark.skipif(not os.path.exists(REF_XML), reason="reference MJCF not mounted")
-def test_committed_asset_matches_a_fresh_compile():
-    from opendog_b200.model.compile import compile_model, load_compiled
-    from opendog_b200.model.mjcf import load_mjcf
-    fresh = compile_model(load_mjcf(REF_XML))
+def test_committed_asset_has_the_reference_model_constants():
+    """The OpenDOG asset against values read off the reference's MJCF (our_robot.xml). Re-deriving the whole asset
+    needs that MJCF and its meshes, which are not part of this repository (tools/compile_model.py does it)."""
+    from opendog_b200.model.compile import load_compiled
     asset = load_compiled("our_robot")
-    assert fresh["nq"] == 15 and fresh["nv"] == 14 and fresh["nu"] == 8 and fresh["ngeom"] == 12
-    for k in ("mass", "ipos", "inertia", "body_pos", "jnt_pos", "jnt_range", "key_qpos", "key_ctrl", "verts",
-              "base_inertia", "base_invweight0", "dof_invweight0"):
-        assert np.allclose(np.asarray(fresh[k], dtype=float), np.asarray(asset[k], dtype=float), rtol=1e-12, atol=1e-15), k
-    assert abs(fresh["base_mass"] + np.sum(fresh["mass"]) - 1.95852) < 1e-12       # SURVEY A.1 total mass
-    assert fresh["act_leg"] == [1, 1, 3, 3, 0, 0, 2, 2]                            # our_robot.xml:99-111
-    assert [g["mj_body_id"] for g in fresh["geoms"] if g["link"] == 1][1::2] == [4, 7, 10, 13]
+    assert asset["nq"] == 15 and asset["nv"] == 14 and asset["nu"] == 8 and asset["ngeom"] == 12
+    assert abs(asset["base_mass"] + np.sum(asset["mass"]) - 1.95852) < 1e-12       # SURVEY A.1 total mass
+    assert asset["act_leg"] == [1, 1, 3, 3, 0, 0, 2, 2]                            # our_robot.xml:99-111
+    assert [g["mj_body_id"] for g in asset["geoms"] if g["link"] == 1][1::2] == [4, 7, 10, 13]
     # floor (condim 3, friction 1) wins the max-mixing against the robot geoms (condim 1, friction .6)
-    assert all(g["condim"] == 3 and g["friction"] == 1.0 and g["margin"] == 0.001 for g in fresh["geoms"])
-    assert fresh["base_armature"] == [0.02] * 6 and fresh["base_frictionloss"] == [0.1] * 6
+    assert all(g["condim"] == 3 and g["friction"] == 1.0 and g["margin"] == 0.001 for g in asset["geoms"])
+    assert asset["base_armature"] == [0.02] * 6 and asset["base_frictionloss"] == [0.1] * 6
 
 
 def test_struct_layouts_match_the_c_headers():
