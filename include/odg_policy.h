@@ -74,7 +74,8 @@ int odg_normalize_advantages(float* adv_dev, long long count, const double* stat
 /* PPO update phase (sim2real/train.py:566-585: `loss.backward()` through `nn.Tanh` + `nn.Linear` of the hidden layers):
  * grad_x = grad_y * (1 - y*y) for a [rows][cols] bf16 activation gradient (torch's tanh_backward) AND, in the same pass
  * over the data, bias_grad[cols] (f32) = the column sums of grad_x = the bias gradient of the Linear that produced the
- * tanh's input. Deterministic (fixed summation order). cols = 8 x a power of two, <= 2048; grad_x must not overlap the inputs.
+ * tanh's input. Deterministic (fixed summation order). cols = 8 x a power of two, <= 2048; grad_y, y and grad_x 16-byte
+ * aligned (ODG_ERR_INVALID otherwise); grad_x must not overlap the inputs.
  * scratch_dev: odg_tanh_backward_bias_scratch_floats(cols) floats of device memory, owned by the caller (so that the call
  * can be captured in a CUDA graph). */
 int odg_tanh_backward_bias_scratch_floats(int cols);
@@ -95,7 +96,7 @@ int odg_ppo_loss(const float* mean_dev, const float* value_dev, const float* log
                  float vf_coef, float ent_coef, float* loss_dev, float* terms_dev, float* grad_mean_dev,
                  float* grad_value_dev, float* grad_log_std_dev, float* scratch_dev, void* stream);
 
-/* PPO update phase, forward: y = tanh(x) for `count` bf16 values (a multiple of 8; 16-byte aligned; y may be x) with the
+/* PPO update phase, forward: y = tanh(x) for `count` bf16 values (a multiple of 8; x and y 16-byte aligned, ODG_ERR_INVALID otherwise; y may be x) with the
  * hardware tanh the rollout kernel's epilogue uses (odg_policy_forward), so that the update-time policy evaluates the same
  * function as the policy that produced logp_old. Replaces nn.Tanh of sim2real/train.py:136-147 on bf16 activations. */
 int odg_tanh_bf16(const void* x_bf16, void* y_bf16, long long count, void* stream);

@@ -704,6 +704,7 @@ int device_of(const void* p) {
   if (cudaPointerGetAttributes(&a, p) != cudaSuccess || a.type != cudaMemoryTypeDevice) { cudaGetLastError(); return -1; }
   return a.device;
 }
+bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 }  // namespace
 
 extern "C" {
@@ -821,6 +822,8 @@ int odg_tanh_backward_bias(const void* grad_y_bf16, const void* y_bf16, void* gr
   if (!grad_y_bf16 || !y_bf16 || !grad_x_bf16 || !bias_grad_dev || !scratch_dev || rows < 1 || cols < 8 || (cols & 7) ||
       groups > kTbBlock || (groups & (groups - 1)))
     return set_error(ODG_ERR_INVALID, "odg_tanh_backward_bias: bad arguments (cols must be 8 x a power of two, <= 2048)");
+  if (!aligned16(grad_y_bf16) || !aligned16(y_bf16) || !aligned16(grad_x_bf16))       // the kernel moves 16-byte vectors
+    return set_error(ODG_ERR_INVALID, "odg_tanh_backward_bias: grad_y, y and grad_x must be 16-byte aligned");
   const int dev = device_of(grad_y_bf16);
   if (dev < 0) return set_error(ODG_ERR_INVALID, "odg_tanh_backward_bias: grad_y is not device memory");
   DevGuard guard(dev);
@@ -857,6 +860,8 @@ int odg_ppo_loss(const float* mean_dev, const float* value_dev, const float* log
 
 int odg_tanh_bf16(const void* x_bf16, void* y_bf16, long long count, void* stream) {
   if (!x_bf16 || !y_bf16 || count < 8 || (count & 7)) return set_error(ODG_ERR_INVALID, "odg_tanh_bf16: bad arguments (count must be a multiple of 8)");
+  if (!aligned16(x_bf16) || !aligned16(y_bf16))                                       // the kernel moves 16-byte vectors
+    return set_error(ODG_ERR_INVALID, "odg_tanh_bf16: x and y must be 16-byte aligned");
   const int dev = device_of(x_bf16);
   if (dev < 0) return set_error(ODG_ERR_INVALID, "odg_tanh_bf16: x is not device memory");
   DevGuard guard(dev);

@@ -96,6 +96,16 @@ def test_c_abi_error_behaviour():
     assert L.odg_ppo_loss(*([None] * 7), 16, 8, 0.2, 0.5, 0.005, *([None] * 7)) == INVALID and b"odg_ppo_loss" in L.odg_last_error()
     assert L.odg_tanh_bf16(None, None, 64, None) == INVALID and b"odg_tanh_bf16" in L.odg_last_error()
     assert L.odg_tanh_backward_bias(None, None, None, None, None, 4, 512, None) == INVALID
+    # the bf16 tensors are moved as 16-byte vectors: a misaligned pointer is refused before any CUDA call (these addresses
+    # are never dereferenced)
+    A16, A8 = C.c_void_p(0x2000), C.c_void_p(0x1008)
+    assert L.odg_tanh_bf16(A8, A16, 64, None) == INVALID and b"16-byte aligned" in L.odg_last_error()
+    assert L.odg_tanh_bf16(A16, A8, 64, None) == INVALID and b"16-byte aligned" in L.odg_last_error()
+    assert L.odg_tanh_bf16(C.c_void_p(0x2002), C.c_void_p(0x2002), 64, None) == INVALID
+    for k in range(3):
+        bf = [A8 if i == k else A16 for i in range(3)]
+        assert L.odg_tanh_backward_bias(*bf, A16, A16, 4, 512, None) == INVALID
+        assert b"odg_tanh_backward_bias" in L.odg_last_error() and b"16-byte aligned" in L.odg_last_error()
     assert L.odg_tanh_backward_bias_scratch_floats(512) >= 512 and L.odg_tanh_backward_bias_scratch_floats(0) == 0
     assert L.odg_ppo_loss_scratch_floats() > 0
     assert L.odg_s2r_step(None, None, None, None, None, None, None, None, None) < 0
