@@ -25,7 +25,8 @@ typedef struct OdgPolicy OdgPolicy;
 #define ODG_POLICY_MAX_ACTION 16
 
 /* Weights of one ActorCritic in the layout of its torch state_dict (float32, device pointers):
- * actor.{0,2,4}.weight [out][in] row-major, actor.{0,2,4}.bias [out], critic.{0,2,4}.*, action_log_std [A]. */
+ * actor.{0,2,4}.weight [out][in] row-major, actor.{0,2,4}.bias [out], critic.{0,2,4}.*, action_log_std [A].
+ * Shapes follow the handle's hidden widths h1 / h2: weight 0 [h1][S], weight 2 [h2][h1], weight 4 [A or 1][h2]. */
 typedef struct OdgPolicyWeights {
   const float* actor_w[3];
   const float* actor_b[3];
@@ -37,6 +38,12 @@ typedef struct OdgPolicyWeights {
 /* Replaces `ActorCritic(state_dim, action_dim, std).to(device)` (sim2real/train.py:533). state_dim <= 64,
  * action_dim <= 16; hidden sizes are the reference's 512 / 256. */
 int odg_policy_create(int state_dim, int action_dim, int device, OdgPolicy** out);
+/* The same with the hidden widths given: (h1, h2) = (512, 256) is odg_policy_create; (1024, 512) is the terrain trainer's
+ * ActorCritic (sim2real/train2.py:149-157, 12 -> 1024 -> 512 -> 8). Any other widths, or state_dim / action_dim out of
+ * range, return ODG_ERR_INVALID before the device is looked at. The 1024 / 512 forward has the same contract as the 512 / 256
+ * one (bf16 operands, fp32 accumulation, the same noise for the same key); its output layer is computed on CUDA cores from
+ * the bf16 hidden-2 values and bf16 weights with fp32 sums. odg_policy_load and odg_policy_forward serve both. */
+int odg_policy_create_hidden(int state_dim, int action_dim, int h1, int h2, int device, OdgPolicy** out);
 void odg_policy_destroy(OdgPolicy* p);
 
 /* Replaces `agent.load_state_dict(...)` / the optimiser's in-place update: converts the fp32 weights to the

@@ -32,12 +32,14 @@ class BatchedQuadrupedEnv:
     50 substeps per policy step); variant "terrain" = sim2real/train2.py:159-411 (8 actions, obs 12, 40 substeps)."""
 
     def __init__(self, num_envs: int, model: str = "our_robot", device=None, auto_reset: bool = True, max_steps: int | None = None,
-                 variant: str = "train", **sim_config):
+                 variant: str = "train", first_env_id: int = 0, **sim_config):
         v = VARIANTS[variant]
         # POLICY_DECISION_DT / timestep: 0.10 / 0.002 = 50 mj_step per policy step (train.py:156), 0.08 / 0.002 = 40 (train2.py:106,178)
+        # first_env_id: global id of environment 0, so that the random streams of a shard are those of the whole batch
         self.sim = BatchedWalkEnv(num_envs, model=model, device=device, info_keys=None, frame_skip=(50, 40)[v], scale_actions=0,
-                                  auto_reset=0, **sim_config)
+                                  auto_reset=0, first_env_id=first_env_id, **sim_config)
         self.L, self.device, self.num_envs = self.sim.L, self.sim.device, self.sim.num_envs
+        self.first_env_id = int(first_env_id)
         self.variant = variant
         cfg = _lib.OdgS2RConfig()
         self.L.odg_s2r_default_config_for(C.byref(cfg), v)
@@ -49,6 +51,7 @@ class BatchedQuadrupedEnv:
         _lib.check(self.L.odg_s2r_create(self.sim._h, C.byref(self.sim._model), C.byref(cfg), C.byref(h)), "odg_s2r_create")
         self._h = h
         self.state_dim, self.action_dim = self.L.odg_s2r_obs_dim(h), self.L.odg_s2r_act_dim(h)     # 22 / 4 (train.py:164), 12 / 8 (train2.py:186)
+        self.obs_dim, self.act_dim = self.state_dim, self.action_dim          # the names opendog_b200.rollout.Rollout reads
         N, dev = num_envs, self.device
         self.obs = torch.empty(N, self.state_dim, device=dev)
         self.reward = torch.empty(N, device=dev)
@@ -77,14 +80,32 @@ class BatchedQuadrupedEnv:
         _lib.check(self.L.odg_s2r_reset(self._h, _ptr(m), _ptr(self.obs), self._stream()), "odg_s2r_reset")
         return self.obs
 
-    def step(self, action: torch.Tensor):
-        a = action.to(device=self.device, dtype=torch.float32).contiguous()
+    def _action(self, action):
+        a = action
+        if a.device != self.device or a.dtype != torch.float32 or not a.is_contiguous():
+            a = a.to(device=self.device, dtype=torch.float32).contiguous()
         if a.shape != (self.num_envs, self.action_dim):
             raise ValueError(f"action must be [{self.num_envs}, {self.action_dim}]")
+        return a
+
+    def step(self, action: torch.Tensor):
+        a = self._action(action)
         _lib.check(self.L.odg_s2r_step(self._h, _ptr(a), _ptr(self.obs), _ptr(self.reward), _ptr(self.done), _ptr(self.reason),
                                        _ptr(self.sim_target_rad), _ptr(self.terminal_obs), self._stream()), "odg_s2r_step")
         info = {"sim_target_rad": self.sim_target_rad, "termination_reason": self.reason, "terminal_obs": self.terminal_obs}
         return self.obs, self.reward, self.done.bool(), info
+
+    def step_into(self, action: torch.Tensor, obs, reward, terminated, truncated):
+        """`step` writing obs / reward straight into caller-owned CUDA tensors (rollout buffers), with the episode ends split
+        the way `BatchedWalkEnv.step_into` reports them: terminated [N] u8 = a termination condition (reason != RUNNING),
+        truncated [N] u8 = the max_steps cap (done with reason RUNNING). `done` and `reason` stay readable on the env.
+        No host synchronisation and no allocation: the call can be captured in a CUDA graph."""
+        a = self._action(action)
+        _lib.check(self.L.odg_s2r_step(self._h, _ptr(a), _ptr(obs), _ptr(reward), _ptr(self.done), _ptr(self.reason),
+                                       None, None, self._stream()), "odg_s2r_step")
+        # a reason other than RUNNING (0) only comes with done = 1, so terminated = min(reason, 1), truncated = done - terminated
+        torch.clamp(self.reason, max=1, out=terminated)
+        torch.sub(self.done, terminated, out=truncated)
 
     def set_bookkeeping(self, counter=None, prev_x=None, cum_pos=None, cum_neg=None, prev_net=None, last_cmd=None):
         def f(t, dt):
@@ -102,9 +123,10 @@ class BatchedTerrainQuadrupedEnv(BatchedQuadrupedEnv):
     next to the physics, not part of it: `hfield_data` / `terrain_height` expose it."""
 
     def __init__(self, num_envs: int, seed: int = 0, first_env_id: int = 0, **kw):
-        super().__init__(num_envs, variant="terrain", **kw)
+        super().__init__(num_envs, variant="terrain", first_env_id=first_env_id, **kw)
         t = C.c_void_p()
-        _lib.check(self.L.odg_terrain_create(num_envs, self.device.index, C.c_uint64(seed), first_env_id, C.byref(t)), "odg_terrain_create")
+        _lib.check(self.L.odg_terrain_create(num_envs, self.device.index, C.c_uint64(seed), self.first_env_id, C.byref(t)),
+                   "odg_terrain_create")
         self._t = t
         self._fields = None
 
@@ -119,11 +141,20 @@ class BatchedTerrainQuadrupedEnv(BatchedQuadrupedEnv):
         _lib.check(self.L.odg_terrain_generate(self._t, _ptr(m), self._stream()), "odg_terrain_generate")
         return super().reset(mask)
 
-    def step(self, action):
-        out = super().step(action)
+    def _regenerate_done(self):
         if self._auto_reset:
             _lib.check(self.L.odg_terrain_generate(self._t, _ptr(self.done), self._stream()), "odg_terrain_generate")
+
+    def step(self, action):
+        out = super().step(action)
+        self._regenerate_done()
         return out
+
+    def step_into(self, action, obs, reward, terminated, truncated):
+        """As `BatchedQuadrupedEnv.step_into`; the environments that were auto-reset get a new field in the same call (so
+        inside a captured CUDA graph too)."""
+        super().step_into(action, obs, reward, terminated, truncated)
+        self._regenerate_done()
 
     @property
     def hfield_data(self) -> torch.Tensor:

@@ -175,6 +175,57 @@ struct MlpParams {
   uint32_t seed_lo, seed_hi, step; const uint32_t* step_base; int first_row;
 };
 
+// obs tile -> bf16 A0 (rows past the batch and columns past S are zero): the 256 epilogue threads, two per row
+__device__ __forceinline__ void load_obs_tile(const MlpParams& P, int K0p, uint8_t* sA0, int tid) {
+  if (tid >= kEpiThreads) return;
+  const int r = tid & (kM - 1), g = blockIdx.x * kM + r;
+  const float* o = P.obs + (size_t)g * P.S;
+  for (int k8 = (tid >> 7) * 8; k8 < K0p; k8 += 16) {
+    uint32_t w[4];
+#pragma unroll
+    for (int i = 0; i < 4; i++) {
+      const int k = k8 + 2 * i;
+      float x0 = (g < P.n && k < P.S) ? o[k] : 0.f;
+      float x1 = (g < P.n && k + 1 < P.S) ? o[k + 1] : 0.f;
+      w[i] = pack_bf16(x0, x1);
+    }
+    *reinterpret_cast<uint4*>(sA0 + canon_off(r, k8, K0p)) = make_uint4(w[0], w[1], w[2], w[3]);
+  }
+}
+
+// Normal(mean, exp(log_std)) of row `grow`: sample + summed log-prob (sim2real/train.py:542-543). Philox4x32-10 keyed by
+// (seed, first_row + grow, step + *step_base, block of 4 action dims, "SAMP"), Box-Muller; shared by both forward kernels,
+// so that the same key draws the same noise whatever the hidden widths.
+__device__ __forceinline__ void sample_row(const MlpParams& P, int grow, const float (&outv)[kNOut]) {
+  const uint32_t step_ctr = P.step + (P.step_base ? __ldg(P.step_base) : 0u);
+  float lp = 0.f;
+#pragma unroll
+  for (int blk = 0; blk < kNOut / 4; blk++) {
+    if (blk * 4 >= P.A) break;
+    uint32_t r[4];
+    odg::philox4x32(P.seed_lo, P.seed_hi, (uint32_t)(P.first_row + grow), step_ctr, (uint32_t)blk, kStreamSample, r);
+#pragma unroll
+    for (int pr = 0; pr < 2; pr++) {                                  // Box-Muller: 2 uniforms -> 2 normals
+      const float u1 = ((float)(r[2 * pr] >> 8) + 1.0f) * 5.9604644775390625e-08f;     // (0, 1]
+      const float u2 = odg::u01(r[2 * pr + 1]);
+      const float rad = sqrtf(-2.0f * logf(u1));
+      float sn, cs; sincosf(6.283185307179586f * u2, &sn, &cs);
+      const float e[2] = { rad * cs, rad * sn };
+#pragma unroll
+      for (int q = 0; q < 2; q++) {
+        const int a = blk * 4 + pr * 2 + q;
+        if (a < P.A) {
+          const float ls = __ldg(P.log_std + a);
+          if (P.mean) P.mean[(size_t)grow * P.A + a] = outv[a];
+          if (P.action) P.action[(size_t)grow * P.A + a] = outv[a] + expf(ls) * e[q];
+          lp += -0.5f * e[q] * e[q] - ls - 0.9189385332046727f;
+        }
+      }
+    }
+  }
+  if (P.logp) P.logp[grow] = lp;
+}
+
 // hidden-layer epilogue of one thread: D[row][c0 .. c0 + ncols) (TMEM, fp32) + bias -> tanh -> bf16 -> A operand tile
 // with `kc_out` columns, written at columns [kofs + c0, ...). Two 32-column TMEM loads are in flight at a time.
 __device__ __forceinline__ void epilogue_hidden(uint32_t taddr_row, int c0, int ncols, const float* __restrict__ bias,
@@ -259,22 +310,7 @@ __global__ void __cluster_dims__(kCluster, 1, 1) __launch_bounds__(kThreads, 1) 
     send(sW3, w3_full, 0, kRingChunks, crank == 0);
   }
   for (int i = tid; i < 2 * kBiasFloats; i += kThreads) s_bias[i] = P.bias[i / kBiasFloats][i % kBiasFloats];
-  // obs tile -> bf16 A0 (rows past the batch and columns past S are zero): 256 threads, two per row
-  if (tid < kEpiThreads) {
-    const int r = tid & (kM - 1), g = blockIdx.x * kM + r;
-    const float* o = P.obs + (size_t)g * P.S;
-    for (int k8 = (tid >> 7) * 8; k8 < K0p; k8 += 16) {
-      uint32_t w[4];
-#pragma unroll
-      for (int i = 0; i < 4; i++) {
-        const int k = k8 + 2 * i;
-        float x0 = (g < P.n && k < P.S) ? o[k] : 0.f;
-        float x1 = (g < P.n && k + 1 < P.S) ? o[k + 1] : 0.f;
-        w[i] = pack_bf16(x0, x1);
-      }
-      *reinterpret_cast<uint4*>(sA0 + canon_off(r, k8, K0p)) = make_uint4(w[0], w[1], w[2], w[3]);
-    }
-  }
+  load_obs_tile(P, K0p, sA0, tid);
   fence_async_smem();
   tc_fence_before();
   __syncthreads();
@@ -354,38 +390,8 @@ __global__ void __cluster_dims__(kCluster, 1, 1) __launch_bounds__(kThreads, 1) 
       mbar_arrive(&acc_free[r]);
     };
     float outv[kNOut];
-    // ---- Normal(mean, exp(log_std)): sample + log-prob  (sim2real/train.py:542-543). Runs in the epilogue warps' idle time
-    // while the critic's layer-2 weights stream in.
-    auto sample_actor = [&]() {
-      if (!(ch == 0 && grow < P.n)) return;
-      const uint32_t step_ctr = P.step + (P.step_base ? __ldg(P.step_base) : 0u);
-      float lp = 0.f;
-#pragma unroll
-      for (int blk = 0; blk < kNOut / 4; blk++) {
-        if (blk * 4 >= P.A) break;
-        uint32_t r[4];
-        odg::philox4x32(P.seed_lo, P.seed_hi, (uint32_t)(P.first_row + grow), step_ctr, (uint32_t)blk, kStreamSample, r);
-#pragma unroll
-        for (int pr = 0; pr < 2; pr++) {                                  // Box-Muller: 2 uniforms -> 2 normals
-          const float u1 = ((float)(r[2 * pr] >> 8) + 1.0f) * 5.9604644775390625e-08f;     // (0, 1]
-          const float u2 = odg::u01(r[2 * pr + 1]);
-          const float rad = sqrtf(-2.0f * logf(u1));
-          float sn, cs; sincosf(6.283185307179586f * u2, &sn, &cs);
-          const float e[2] = { rad * cs, rad * sn };
-#pragma unroll
-          for (int q = 0; q < 2; q++) {
-            const int a = blk * 4 + pr * 2 + q;
-            if (a < P.A) {
-              const float ls = __ldg(P.log_std + a);
-              if (P.mean) P.mean[(size_t)grow * P.A + a] = outv[a];
-              if (P.action) P.action[(size_t)grow * P.A + a] = outv[a] + expf(ls) * e[q];
-              lp += -0.5f * e[q] * e[q] - ls - 0.9189385332046727f;
-            }
-          }
-        }
-      }
-      if (P.logp) P.logp[grow] = lp;
-    };
+    // the actor's sample + log-prob: runs in the epilogue warps' idle time while the critic's layer-2 weights stream in
+    auto sample_actor = [&]() { if (ch == 0 && grow < P.n) sample_row(P, grow, outv); };
     if (tid == 0) MLP_STAMP(0);
     for (int net = 0; net < 2; net++) {
       const float* b1 = s_bias + net * kBiasFloats; const float* b2 = b1 + kH1; const float* b3 = b2 + kH2;
@@ -427,6 +433,228 @@ __global__ void __cluster_dims__(kCluster, 1, 1) __launch_bounds__(kThreads, 1) 
   cluster_sync_all();                                  // no CTA leaves while its peer may still signal its barriers
 }
 
+// ---------------------------------------------------------------------------------------------- k_mlp_wide
+// The terrain trainer's ActorCritic (sim2real/train2.py:149-157): Linear(S,1024)-tanh -> Linear(1024,512)-tanh -> head,
+// with k_mlp's contract (bf16 operands, fp32 accumulation in TMEM, tanh.approx on the hidden layers, tanhf on the actor
+// head, sample_row). A 128 x 1024 bf16 hidden-1 tile (256 KB) does not fit shared memory, so hidden 1 is never stored
+// whole. Layer 2 runs as two N = 256 halves, each accumulating in TMEM columns 0-255; for each half hidden 1 is recomputed
+// in 128-column chunks (layer 1 has K = K0p <= 64: K0p / (K0p + 512) more FLOPs, 3 % at the terrain trainer's S = 12, 11 % at S = 64) into TMEM columns 256-383 / 384-511 (ping-pong), and the
+// epilogue drains each chunk into one of two 32 KB bf16 buffers, the A operand of that chunk's layer-2 MMAs. The head
+// (K = 512; A or 1 outputs) runs on CUDA cores inside the hidden-2 epilogue: bf16-rounded hidden 2 times bf16 W3, fp32
+// sums, so no 128 KB hidden-2 tile either. Work unit U = (network, half, chunk), 32 per CTA; the MMA issue order is
+// L1(0), L1(1), L2(0), L1(2), L2(1), ... so that the epilogue drains chunk U + 1 while the layer-2 MMAs of chunk U run.
+constexpr int kWH1 = 1024, kWH2 = 512;
+constexpr int kWChunkCols = 128;                                 // hidden-1 columns per recomputed chunk (N of layer 1)
+constexpr int kWChunks = kWH1 / kWChunkCols;                     // 8 chunks per layer-2 half
+constexpr int kWHalves = kWH2 / 256;                             // 2 layer-2 halves of N = 256
+constexpr int kWUnitsPerNet = kWHalves * kWChunks, kWUnits = 2 * kWUnitsPerNet;
+constexpr int kWL2PerUnit = kWChunkCols / kK2Chunk;              // 4 W2 stages (256 x 32) per unit
+constexpr int kWW2Chunks = kWHalves * (kWH1 / kK2Chunk);         // 64 packed W2 chunks per network
+constexpr int kWNumChunks = kWChunks + kWW2Chunks + 1;           // + W3 = 73 packed chunks per network
+constexpr int kWW3Bytes = kWH2 * kNOut * 2;                      // 16 KB: W3 as [512][16] bf16 (a hidden-2 unit's head weights)
+constexpr int kWH1Bytes = kM * kWChunkCols * 2;                  // 32 KB hidden-1 chunk
+constexpr int kWOffA0 = 0, kWOffH1 = kWOffA0 + kA0Bytes, kWOffW = kWOffH1 + 2 * kWH1Bytes;
+constexpr int kWOffW3 = kWOffW + kStages * kWBufBytes;          // both networks' W3, loaded once
+constexpr int kWOffX = kWOffW3 + 2 * kWW3Bytes;                 // head partial sums of the second column half, [2][128][16] f32
+constexpr int kWOffBar = kWOffX + 2 * kM * kNOut * 4;
+constexpr int kWBiasFloats = kWH1 + kWH2 + kNOut;               // per network: b1 | b2 | b3
+constexpr int kWOffBias = kWOffBar + 256;
+constexpr int kWSmemBytes = kWOffBias + 2 * kWBiasFloats * 4;
+static_assert(kWSmemBytes <= 227 * 1024, "k_mlp_wide: shared memory over the 227 KB a block may use");
+
+// packed chunks of one network: W1 [0, 8) (128 x K0p), W2 [8, 72) (256 x 32: half h, K-chunk k at 8 + 32 h + k), W3 72
+__host__ __device__ inline int wide_chunk_bytes(int c, int K0p) { return c < kWChunks ? kWChunkCols * K0p * 2 : kWBufBytes; }
+__host__ __device__ inline int wide_chunk_offset(int c, int K0p) {
+  return c <= kWChunks ? c * kWChunkCols * K0p * 2 : kWChunks * kWChunkCols * K0p * 2 + (c - kWChunks) * kWBufBytes;
+}
+
+// hidden-2 epilogue of one thread with the head folded in: for the 128 columns [c0, c0 + 128) of a layer-2 half,
+// h = bf16(tanh(D + b2)) (the value the next layer's bf16 operand would hold), acc[a] += h * W3[a][col] for a < NO
+template <int NO>
+__device__ __forceinline__ void epilogue_head(uint32_t taddr_row, int c0, const float* __restrict__ bias, const uint8_t* w3,
+                                              float (&acc)[kNOut]) {
+  for (int cb = c0; cb < c0 + 128; cb += 32) {
+    uint32_t v[32];
+    tmem_ld32_nowait(taddr_row + cb, v);
+    tmem_ld_wait();
+#pragma unroll
+    for (int i = 0; i < 32; i++) {
+      const int col = cb + i;
+      const float h = __bfloat162float(__float2bfloat16_rn(tanh_fast(__uint_as_float(v[i]) + bias[col])));
+      const __nv_bfloat162* w = reinterpret_cast<const __nv_bfloat162*>(w3 + col * kNOut * 2);
+#pragma unroll
+      for (int a = 0; a < NO; a += 2) {
+        const float2 wf = __bfloat1622float2(w[a / 2]);
+        acc[a] = fmaf(h, wf.x, acc[a]);
+        if (a + 1 < NO) acc[a + 1] = fmaf(h, wf.y, acc[a + 1]);
+      }
+    }
+  }
+}
+
+// Barriers (single-CTA mbarriers unless noted):
+//   w_full[s] / w_free[s]   weight stage s landed / its MMAs retired in BOTH CTAs of the cluster (as in k_mlp)
+//   w3_full                 both networks' W3 landed (one multicast copy per network)
+//   l1_full[b]              layer-1 MMAs of a chunk into TMEM region 256 + 128 b retired
+//   h1_ready[b]             the epilogue drained region b and wrote hidden-1 buffer b (256 arrivals)
+//   h1_free[b]              the layer-2 MMAs reading hidden-1 buffer b retired
+//   acc2_full / acc2_free   a layer-2 half in TMEM columns 0-255 is complete / drained by the epilogue
+__global__ void __cluster_dims__(kCluster, 1, 1) __launch_bounds__(kThreads, 1) k_mlp_wide(const MlpParams P) {
+  extern __shared__ __align__(1024) uint8_t smem[];
+  uint8_t* sA0 = smem + kWOffA0; uint8_t* sH1 = smem + kWOffH1; uint8_t* sW = smem + kWOffW; uint8_t* sW3 = smem + kWOffW3;
+  float* sX = reinterpret_cast<float*>(smem + kWOffX);
+  uint64_t* w_full = reinterpret_cast<uint64_t*>(smem + kWOffBar);      // [kStages]
+  uint64_t* w_free = w_full + kStages;                                  // [kStages]
+  uint64_t* l1_full = w_free + kStages;                                 // [2]
+  uint64_t* h1_ready = l1_full + 2;                                     // [2]
+  uint64_t* h1_free = h1_ready + 2;                                     // [2]
+  uint64_t* acc2_full = h1_free + 2;
+  uint64_t* acc2_free = acc2_full + 1;
+  uint64_t* w3_full = acc2_free + 1;
+  uint32_t* s_tmem = reinterpret_cast<uint32_t*>(w3_full + 1);
+  float* s_bias = reinterpret_cast<float*>(smem + kWOffBias);
+  const int tid = threadIdx.x, warp = tid >> 5;
+  const int K0p = P.K0p;
+
+  if (tid == 0) {
+    for (int i = 0; i < kStages; i++) { mbar_init(&w_full[i], 1); mbar_init(&w_free[i], kCluster); }
+    for (int i = 0; i < 2; i++) { mbar_init(&l1_full[i], 1); mbar_init(&h1_ready[i], kEpiThreads); mbar_init(&h1_free[i], 1); }
+    mbar_init(acc2_full, 1); mbar_init(acc2_free, kEpiThreads); mbar_init(w3_full, 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  if (warp == 0) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" :: "r"(smem_u32(s_tmem)), "r"(512) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  }
+  __syncthreads();
+  cluster_sync_all();
+  constexpr uint16_t kAllCtas = (uint16_t)((1u << kCluster) - 1);
+  const uint32_t crank = cluster_ctarank();
+  for (int i = tid; i < 2 * kWBiasFloats; i += kThreads) s_bias[i] = P.bias[i / kWBiasFloats][i % kWBiasFloats];
+  load_obs_tile(P, K0p, sA0, tid);
+  fence_async_smem();
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem = *s_tmem;
+
+  if (tid == kProducerTid) {
+    // ---- weight producer: both W3 once, then the ring in the issuer's order (W1 of unit U + 1 before the W2 of unit U)
+    mbar_expect_tx(w3_full, 2u * kWW3Bytes);
+    for (int net = 0; net < 2; net++)
+      if ((uint32_t)(net % kCluster) == crank)
+        bulk_g2s_multicast(sW3 + net * kWW3Bytes, P.wpack[net] + wide_chunk_offset(kWNumChunks - 1, K0p), kWW3Bytes, w3_full, kAllCtas);
+    int c = 0;
+    auto push = [&](int net, int packed) {
+      const int st = c % kStages;
+      if (c >= kStages) mbar_wait(&w_free[st], (uint32_t)((c / kStages - 1) & 1));       // freed by every CTA of the cluster
+      const uint32_t bytes = (uint32_t)wide_chunk_bytes(packed, K0p);
+      mbar_expect_tx(&w_full[st], bytes);
+      if ((uint32_t)(c % kCluster) == crank)
+        bulk_g2s_multicast(sW + st * kWBufBytes, P.wpack[net] + wide_chunk_offset(packed, K0p), bytes, &w_full[st], kAllCtas);
+      c++;
+    };
+    push(0, 0);
+    for (int U = 0; U < kWUnits; U++) {
+      if (U + 1 < kWUnits) push((U + 1) / kWUnitsPerNet, (U + 1) % kWChunks);
+      const int net = U / kWUnitsPerNet, nh = (U / kWChunks) % kWHalves, j = U % kWChunks;
+      for (int q = 0; q < kWL2PerUnit; q++) push(net, kWChunks + nh * (kWH1 / kK2Chunk) + j * kWL2PerUnit + q);
+    }
+  } else if (tid == kIssuerTid) {
+    // ---- MMA issuer
+    int c = 0;
+    uint32_t ph_ready[2] = { 0, 0 }, ph_acc2_free = 0;
+    auto mma_stage = [&](uint32_t a_saddr, uint32_t a_sbo, int ksteps, uint32_t b_sbo, uint32_t dcol, int ncols, bool accumulate) {
+      const int st = c % kStages;
+      mbar_wait(&w_full[st], (uint32_t)((c / kStages) & 1));
+      tc_fence_after();
+      const uint32_t b_saddr = smem_u32(sW + st * kWBufBytes), idesc = make_idesc(kM, ncols);
+      for (int k = 0; k < ksteps; k++)
+        umma_bf16(tmem + dcol, make_desc(a_saddr + k * 256, 128, a_sbo), make_desc(b_saddr + k * 256, 128, b_sbo), idesc,
+                  (accumulate || k > 0) ? 1u : 0u);
+      umma_commit_multicast(&w_free[st], kAllCtas);
+      c++;
+    };
+    // layer 1 of unit U -> TMEM region U & 1. Its previous user, unit U - 2, was drained: the issuer waited for h1_ready of
+    // U - 2 before issuing L2(U - 2), which precedes this call
+    auto layer1 = [&](int U) {
+      const uint32_t sbo = (uint32_t)(K0p >> 3) * 128u;
+      mma_stage(smem_u32(sA0), sbo, K0p / 16, sbo, 256u + (uint32_t)(U & 1) * kWChunkCols, kWChunkCols, false);
+      umma_commit(&l1_full[U & 1]);
+    };
+    layer1(0);
+    for (int U = 0; U < kWUnits; U++) {
+      if (U + 1 < kWUnits) layer1(U + 1);
+      const int b = U & 1, j = U % kWChunks;
+      mbar_wait(&h1_ready[b], ph_ready[b]); ph_ready[b] ^= 1;
+      if (j == 0 && U > 0) { mbar_wait(acc2_free, ph_acc2_free); ph_acc2_free ^= 1; }
+      tc_fence_after();
+      for (int q = 0; q < kWL2PerUnit; q++)
+        mma_stage(smem_u32(sH1 + b * kWH1Bytes) + q * (kK2Chunk / 8) * 128, (uint32_t)(kWChunkCols >> 3) * 128u, kK2Chunk / 16,
+                  (uint32_t)(kK2Chunk >> 3) * 128u, 0u, 256, j > 0 || q > 0);
+      umma_commit(&h1_free[b]);
+      if (j == kWChunks - 1) umma_commit(acc2_full);
+    }
+  } else if (tid < kEpiThreads) {
+    // ---- epilogue warpgroups: thread = (row, column half)
+    const int row = tid & (kM - 1), ch = tid >> 7;
+    const int grow = blockIdx.x * kM + row;
+    const uint32_t tmem_row = tmem + ((uint32_t)((warp & 3) * 32) << 16);
+    uint32_t ph_l1[2] = { 0, 0 }, ph_free[2] = { 0, 0 }, ph_acc2 = 0;
+    float acc[kNOut], outv[kNOut];
+    for (int U = 0; U < kWUnits; U++) {
+      const int net = U / kWUnitsPerNet, nh = (U / kWChunks) % kWHalves, j = U % kWChunks, b = U & 1;
+      const float* b1 = s_bias + net * kWBiasFloats; const float* b2 = b1 + kWH1; const float* b3 = b2 + kWH2;
+      if (U % kWUnitsPerNet == 0) {
+#pragma unroll
+        for (int a = 0; a < kNOut; a++) acc[a] = 0.f;
+      }
+      mbar_wait(&l1_full[b], ph_l1[b]); ph_l1[b] ^= 1;
+      if (U >= 2) { mbar_wait(&h1_free[b], ph_free[b]); ph_free[b] ^= 1; }          // L2(U - 2) no longer reads buffer b
+      tc_fence_after();
+      epilogue_hidden(tmem_row + 256 + b * kWChunkCols, ch * 64, 64, b1 + j * kWChunkCols, sH1 + b * kWH1Bytes, kWChunkCols, 0, row);
+      tc_fence_before();
+      fence_async_smem();
+      mbar_arrive(&h1_ready[b]);
+      if (j != kWChunks - 1) continue;
+      // ---- a layer-2 half is complete: hidden 2 + head partial sums
+      mbar_wait(acc2_full, ph_acc2); ph_acc2 ^= 1;
+      tc_fence_after();
+      if (U == kWChunks - 1) mbar_wait(w3_full, 0u);
+      const uint8_t* w3 = sW3 + net * kWW3Bytes + nh * 256 * kNOut * 2;
+      if (net == 1) epilogue_head<1>(tmem_row, ch * 128, b2 + nh * 256, w3, acc);
+      else if (P.A <= 8) epilogue_head<8>(tmem_row, ch * 128, b2 + nh * 256, w3, acc);
+      else epilogue_head<16>(tmem_row, ch * 128, b2 + nh * 256, w3, acc);
+      tc_fence_before();
+      mbar_arrive(acc2_free);
+      if (nh != kWHalves - 1) continue;
+      // ---- the network is complete: add the two column halves' partial sums (fixed order), head bias, output
+      float* x = sX + (net * kM + row) * kNOut;
+      if (ch == 1) {
+#pragma unroll
+        for (int a = 0; a < kNOut; a++) x[a] = acc[a];
+      }
+      asm volatile("bar.sync 1, %0;" :: "r"(kEpiThreads) : "memory");     // the 256 epilogue threads only
+      if (ch == 0) {
+        if (net == 0) {
+#pragma unroll
+          for (int a = 0; a < kNOut; a++) outv[a] = tanhf(acc[a] + x[a] + b3[a]);          // actor: Tanh head
+          if (grow < P.n) sample_row(P, grow, outv);
+        } else if (grow < P.n && P.value) {
+          P.value[grow] = acc[0] + x[0] + b3[0];
+        }
+      }
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 0) {
+    tc_fence_after();
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "r"(512) : "memory");
+  }
+  cluster_sync_all();                                  // no CTA leaves while its peer may still signal its barriers
+}
+
 // fp32 [out][in] weights -> bf16 chunks. One thread per destination element pair.
 __global__ void k_pack(const float* __restrict__ w0, const float* __restrict__ w1, const float* __restrict__ w2,
                        int S, int nout, int K0p, uint8_t* __restrict__ dst) {
@@ -441,11 +669,38 @@ __global__ void k_pack(const float* __restrict__ w0, const float* __restrict__ w
   else { if (r < nout) v = w2[(size_t)r * kH2 + k]; }
   *reinterpret_cast<__nv_bfloat16*>(dst + chunk_offset(c, K0p) + canon_off(r, k, d.kc)) = __float2bfloat16_rn(v);
 }
-__global__ void k_pack_bias(const float* b0, const float* b1, const float* b2, int nout, float* dst) {
+// the same for k_mlp_wide's chunks (wide_chunk_offset); W3 goes to [512][16] for the CUDA-core head
+__global__ void k_pack_wide(const float* __restrict__ w0, const float* __restrict__ w1, const float* __restrict__ w2,
+                            int S, int nout, int K0p, uint8_t* __restrict__ dst) {
+  const int c = blockIdx.y;
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  float v = 0.f;
+  int off;
+  if (c < kWChunks) {                                                   // W1 rows [128 c, 128 c + 128)
+    if (e >= kWChunkCols * K0p) return;
+    const int r = e / K0p, k = e % K0p;
+    if (k < S) v = w0[(size_t)(c * kWChunkCols + r) * S + k];
+    off = canon_off(r, k, K0p);
+  } else if (c < kWChunks + kWW2Chunks) {                               // W2 rows of half h, K-chunk kq
+    if (e >= 256 * kK2Chunk) return;
+    const int q = c - kWChunks, h = q / (kWH1 / kK2Chunk), kq = q % (kWH1 / kK2Chunk);
+    const int r = e / kK2Chunk, k = e % kK2Chunk;
+    v = w1[(size_t)(h * 256 + r) * kWH1 + kq * kK2Chunk + k];
+    off = canon_off(r, k, kK2Chunk);
+  } else {                                                              // W3 transposed: [hidden-2 unit][output]
+    if (e >= kWH2 * kNOut) return;
+    const int k = e / kNOut, a = e % kNOut;
+    if (a < nout) v = w2[(size_t)a * kWH2 + k];
+    off = e * 2;
+  }
+  *reinterpret_cast<__nv_bfloat16*>(dst + wide_chunk_offset(c, K0p) + off) = __float2bfloat16_rn(v);
+}
+// b1 [h1] | b2 [h2] | b3 [nout] zero-padded to 16
+__global__ void k_pack_bias(const float* b0, const float* b1, const float* b2, int h1, int h2, int nout, float* dst) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < kH1) dst[i] = b0[i];
-  else if (i < kH1 + kH2) dst[i] = b1[i - kH1];
-  else if (i < kH1 + kH2 + kNOut) { const int a = i - kH1 - kH2; dst[i] = a < nout ? b2[a] : 0.f; }
+  if (i < h1) dst[i] = b0[i];
+  else if (i < h1 + h2) dst[i] = b1[i - h1];
+  else if (i < h1 + h2 + kNOut) { const int a = i - h1 - h2; dst[i] = a < nout ? b2[a] : 0.f; }
 }
 
 // ---------------------------------------------------------------------------------------------- GAE
@@ -684,6 +939,7 @@ __global__ void __launch_bounds__(256) k_tanh_bf16(const uint4* x, uint4* y, lon
 
 struct OdgPolicy {
   int device = 0, S = 0, A = 0, K0p = 0;
+  bool wide = false;                     // hidden 1024 / 512 (k_mlp_wide) instead of 512 / 256 (k_mlp)
   uint8_t* d_wpack[2] = { nullptr, nullptr };
   float* d_bias[2] = { nullptr, nullptr };
   float* d_log_std = nullptr;
@@ -710,8 +966,15 @@ bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 
 extern "C" {
 
 int odg_policy_create(int state_dim, int action_dim, int device, OdgPolicy** out) {
+  return odg_policy_create_hidden(state_dim, action_dim, kH1, kH2, device, out);
+}
+
+int odg_policy_create_hidden(int state_dim, int action_dim, int h1, int h2, int device, OdgPolicy** out) {
   if (!out || state_dim < 1 || state_dim > ODG_POLICY_MAX_STATE || action_dim < 1 || action_dim > ODG_POLICY_MAX_ACTION)
     return set_error(ODG_ERR_INVALID, "odg_policy_create: state_dim must be in [1,64], action_dim in [1,16]");
+  const bool wide = h1 == kWH1 && h2 == kWH2;
+  if (!wide && !(h1 == kH1 && h2 == kH2))
+    return set_error(ODG_ERR_INVALID, "odg_policy_create_hidden: hidden widths must be (512, 256) or (1024, 512)");
   *out = nullptr;
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
@@ -720,11 +983,12 @@ int odg_policy_create(int state_dim, int action_dim, int device, OdgPolicy** out
   DevGuard guard(device);
   OdgPolicy* p = new (std::nothrow) OdgPolicy();
   if (!p) return set_error(ODG_ERR_ALLOC, "out of host memory");
-  p->device = device; p->S = state_dim; p->A = action_dim; p->K0p = (state_dim + 15) / 16 * 16;
-  p->wpack_bytes = (size_t)chunk_offset(kNumChunks, p->K0p);
+  p->device = device; p->S = state_dim; p->A = action_dim; p->K0p = (state_dim + 15) / 16 * 16; p->wide = wide;
+  p->wpack_bytes = (size_t)(wide ? wide_chunk_offset(kWNumChunks, p->K0p) : chunk_offset(kNumChunks, p->K0p));
+  const size_t bias_floats = wide ? kWBiasFloats : kBiasFloats;
   for (int net = 0; net < 2; net++) {
     if (cudaMalloc(&p->d_wpack[net], p->wpack_bytes) != cudaSuccess ||
-        cudaMalloc(&p->d_bias[net], (kH1 + kH2 + kNOut) * sizeof(float)) != cudaSuccess) {
+        cudaMalloc(&p->d_bias[net], bias_floats * sizeof(float)) != cudaSuccess) {
       odg_policy_destroy(p); return set_error(ODG_ERR_ALLOC, "cudaMalloc(policy) failed");
     }
   }
@@ -732,7 +996,8 @@ int odg_policy_create(int state_dim, int action_dim, int device, OdgPolicy** out
     odg_policy_destroy(p); return set_error(ODG_ERR_ALLOC, "cudaMalloc(policy) failed");
   }
   CUDA_TRY(cudaMemset(p->d_log_std, 0, ODG_POLICY_MAX_ACTION * sizeof(float)));
-  CUDA_TRY(cudaFuncSetAttribute(k_mlp, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
+  if (wide) CUDA_TRY(cudaFuncSetAttribute(k_mlp_wide, cudaFuncAttributeMaxDynamicSharedMemorySize, kWSmemBytes));
+  else CUDA_TRY(cudaFuncSetAttribute(k_mlp, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
   *out = p;
   return ODG_OK;
 }
@@ -755,9 +1020,10 @@ int odg_policy_load(OdgPolicy* p, const OdgPolicyWeights* w, void* stream) {
     for (int i = 0; i < 3; i++) if (!W[i] || !B[i]) return set_error(ODG_ERR_INVALID, "odg_policy_load: missing weight pointer");
     const int nout = net == 0 ? p->A : 1;
     const int max_elems = kWBufBytes / 2;                            // elements of the largest chunk
-    dim3 grid((max_elems + 255) / 256, kNumChunks);
-    k_pack<<<grid, 256, 0, st>>>(W[0], W[1], W[2], p->S, nout, p->K0p, p->d_wpack[net]);
-    k_pack_bias<<<(kH1 + kH2 + kNOut + 255) / 256, 256, 0, st>>>(B[0], B[1], B[2], nout, p->d_bias[net]);
+    const int h1 = p->wide ? kWH1 : kH1, h2 = p->wide ? kWH2 : kH2;
+    if (p->wide) k_pack_wide<<<dim3((max_elems + 255) / 256, kWNumChunks), 256, 0, st>>>(W[0], W[1], W[2], p->S, nout, p->K0p, p->d_wpack[net]);
+    else k_pack<<<dim3((max_elems + 255) / 256, kNumChunks), 256, 0, st>>>(W[0], W[1], W[2], p->S, nout, p->K0p, p->d_wpack[net]);
+    k_pack_bias<<<(h1 + h2 + kNOut + 255) / 256, 256, 0, st>>>(B[0], B[1], B[2], h1, h2, nout, p->d_bias[net]);
     p->launches += 2;
   }
   if (w->action_log_std)
@@ -777,7 +1043,8 @@ int odg_policy_forward(OdgPolicy* p, const float* obs_dev, int n, float* mean_de
   P.log_std = p->d_log_std; P.mean = mean_dev; P.value = value_dev; P.action = action_dev; P.logp = logp_dev;
   P.seed_lo = (uint32_t)seed; P.seed_hi = (uint32_t)(seed >> 32); P.step = step; P.step_base = step_base_dev; P.first_row = first_row_id;
   const int ctas = ((n + kM - 1) / kM + kCluster - 1) / kCluster * kCluster;       // whole clusters; surplus rows are masked
-  k_mlp<<<ctas, kThreads, kSmemBytes, static_cast<cudaStream_t>(stream)>>>(P);
+  if (p->wide) k_mlp_wide<<<ctas, kThreads, kWSmemBytes, static_cast<cudaStream_t>(stream)>>>(P);
+  else k_mlp<<<ctas, kThreads, kSmemBytes, static_cast<cudaStream_t>(stream)>>>(P);
   p->launches++;
   CUDA_TRY(cudaGetLastError());
   return ODG_OK;

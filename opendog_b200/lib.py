@@ -20,7 +20,7 @@ SYMBOLS = [
     "odg_get_env_state", "odg_set_env_state", "odg_launch_count", "odg_last_error", "odg_version", "odg_set_frame_skip",
     "odg_step_host",
     # rollout / policy entry points (include/odg_policy.h)
-    "odg_policy_create", "odg_policy_destroy", "odg_policy_load", "odg_policy_forward", "odg_gae",
+    "odg_policy_create", "odg_policy_create_hidden", "odg_policy_destroy", "odg_policy_load", "odg_policy_forward", "odg_gae",
     "odg_normalize_advantages", "odg_policy_launch_count", "odg_tanh_backward_bias", "odg_tanh_backward_bias_scratch_floats",
     "odg_ppo_loss", "odg_ppo_loss_scratch_floats", "odg_tanh_bf16",
     # QuadrupedEnv surface (include/odg_sim2real.h)
@@ -98,6 +98,7 @@ def load():
     L.odg_get_env_state.argtypes = [_vp] * 8
     L.odg_set_env_state.argtypes = [_vp] * 8
     L.odg_policy_create.argtypes = [C.c_int, C.c_int, C.c_int, C.POINTER(_vp)]
+    L.odg_policy_create_hidden.argtypes = [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(_vp)]
     L.odg_policy_destroy.argtypes = [_vp]
     L.odg_policy_destroy.restype = None
     L.odg_policy_load.argtypes = [_vp, C.POINTER(OdgPolicyWeights), _vp]

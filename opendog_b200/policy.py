@@ -2,7 +2,7 @@
 
 `ActorCriticB200` keeps the parameters in the reference's own `state_dict` layout (`actor.{0,2,4}.{weight,bias}`,
 `critic.*`, `action_log_std`), so a reference `.pth` loads unchanged and a torch optimiser can update them. The
-batched forward used while collecting rollouts (`act`) is libodgsim's fused tcgen05 kernel (include/odg_policy.h);
+batched forward used while collecting rollouts (`act`) is one of libodgsim's fused tcgen05 kernels (include/odg_policy.h);
 `evaluate` — the differentiable forward the PPO/A2C update needs — stays plain torch autograd, as in the reference.
 """
 from __future__ import annotations
@@ -21,10 +21,12 @@ def _ptr(t):
 
 
 class ActorCriticB200(nn.Module):
-    """`hidden` = the two hidden widths: (512, 256) is sim2real/train.py:135-149 and the benchmark policy — its rollout-time
-    forward is the fused tcgen05 kernel; (1024, 512) is the terrain trainer's network (sim2real/train2.py:151-153), whose
-    128 x 1024 bf16 hidden tile does not fit one SM's shared memory next to the weight stages: `act` then runs the same
-    arithmetic (bf16 operands, fp32 accumulation) as library GEMMs through torch, on the device, with the same outputs."""
+    """`hidden` = the two hidden widths. (512, 256) is sim2real/train.py:135-149 and the benchmark policy; (1024, 512) is
+    the terrain trainer's network (sim2real/train2.py:151-153). For both, the rollout-time forward (`act`) is one fused
+    tcgen05 kernel launch with the sampling in its epilogue (include/odg_policy.h): the noise is Philox keyed by
+    (seed, global row id, step), so sharded and graphed rollouts draw the same noise, and the hidden layers use the
+    hardware tanh the update phase's `linear_tanh` uses. Other widths (the reference's older 22-256-256-4 checkpoints) run
+    `_act_library`: the same arithmetic as library GEMMs through torch, with noise from a torch generator."""
 
     def __init__(self, state_dim: int, action_dim: int, action_std_init: float = 0.4, device=None, seed: int = 0,
                  hidden=(512, 256)):
@@ -37,7 +39,7 @@ class ActorCriticB200(nn.Module):
         self.state_dim, self.action_dim, self.seed = state_dim, action_dim, seed
         h1, h2 = int(hidden[0]), int(hidden[1])
         self.hidden = (h1, h2)
-        self.fused = self.hidden == (512, 256)
+        self.fused = self.hidden in ((512, 256), (1024, 512))          # the widths libodgsim's forward kernels cover
         self.actor = nn.Sequential(nn.Linear(state_dim, h1), nn.Tanh(), nn.Linear(h1, h2), nn.Tanh(),
                                    nn.Linear(h2, action_dim), nn.Tanh())
         self.critic = nn.Sequential(nn.Linear(state_dim, h1), nn.Tanh(), nn.Linear(h1, h2), nn.Tanh(),
@@ -51,7 +53,8 @@ class ActorCriticB200(nn.Module):
         self._gen.manual_seed(seed)
         if self.fused:
             h = C.c_void_p()
-            _lib.check(self.L.odg_policy_create(state_dim, action_dim, self.dev.index, C.byref(h)), "odg_policy_create")
+            _lib.check(self.L.odg_policy_create_hidden(state_dim, action_dim, h1, h2, self.dev.index, C.byref(h)),
+                       "odg_policy_create_hidden")
             self._h = h
         self._step = 0
         self.sync_weights()
@@ -119,8 +122,8 @@ class ActorCriticB200(nn.Module):
 
     @torch.no_grad()
     def _act_library(self, o, sample, out):
-        """Rollout-time forward for hidden sizes the fused kernel does not cover: bf16 operands, fp32 accumulation, on
-        the device (cuBLAS through torch). Same outputs as the kernel path; the noise comes from a torch generator."""
+        """Rollout-time forward for hidden sizes neither fused kernel covers: bf16 operands, fp32 accumulation, on the
+        device (cuBLAS through torch). The noise comes from a torch generator, not the kernels' keyed Philox stream."""
         with torch.autocast("cuda", dtype=torch.bfloat16):
             mean = self.actor(o).float()
             value = self.critic(o).float().squeeze(-1)
