@@ -451,7 +451,8 @@ ODG_DEV int cone_eval(V3 z, float Dn, float Dt, float mu, float fri, float dmk, 
 // sticking-zone quadratic q1 + alpha q2, the cone-surface stiffness Dm and mu. `cone_line_eval` (every pass of the search)
 // adds d/dalpha cost(z0 + al[k] dz) at W step lengths from those nine numbers alone — no per-slot constants, no vector
 // arithmetic in the search's inner loop. Branch-free zone selection so the W evaluations interleave. The line search only
-// positions the step; the solution the iteration converges to does not depend on it.
+// positions the step and sets how many iterations the solve takes (tests/test_solver_optimality.py); with one or two
+// passes it can stall at the iteration cap (odg_prep.h rejects ls_iterations < 3).
 struct LineCoef { float N0, Nd, cA, cB, cC, q1, q2, Dm, mu; };
 ODG_DEV LineCoef cone_line_prep(V3 z0, V3 dz, float Dn, float Dt, float mu, float fri, float dmk, int condim) {
   // a frictionless (condim 1) row is the same cone with no tangential part: fri = Dt = 0 gives T = 0, zone = (N >= 0 ?

@@ -328,7 +328,14 @@ inline std::string prepare(const OdgModel& m, const OdgEnvConfig& cfg, uint64_t 
   C.obs_dim = cfg.task == ODG_TASK_JUMP ? 9 + m.nu : (C.obs_layout ? 12 : 9) + 3 * m.nu;
   C.first_env_id = cfg.first_env_id; C.tol = cfg.solver_tolerance; C.ls_tol = cfg.ls_tolerance; C.noise = cfg.reset_noise_scale;
   C.seed_lo = (uint32_t)seed; C.seed_hi = (uint32_t)(seed >> 32);
-  if (cfg.frame_skip < 1 || cfg.solver_iterations < 1 || cfg.ls_iterations < 1) return "bad config";
+  if (cfg.frame_skip < 1 || cfg.solver_iterations < 1) return "bad config";
+  // one pass evaluates only {0.25, 0.5, 1, 2}: a zero of phi' below 0.25 (a stiff row switching on next to the iterate)
+  // then gets the chord across the kink on every iteration and the solve reaches the iteration cap unconverged. Two
+  // passes leave the ladder no pass to refine its bracket in, and states of both models still stall at the cap far from
+  // the optimum. In the GPU-sized state sets of tests/test_solver_optimality.py (same indices on the B200 and in the
+  // host emulator): OpenDOG rollout state 1729 at ls_tolerance 0.01 (gap 7e9 x its float32 floor), OpenDOG rest state
+  // 2457 at 0.1 (1.5e9 x), Go1 rollout state 447 at 0.5 (3.9e9 x)
+  if (cfg.ls_iterations < 3) return "ls_iterations must be >= 3 (fewer passes cannot resolve steps below 0.25)";
   return "";
 }
 
