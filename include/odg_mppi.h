@@ -46,6 +46,36 @@ int odg_mppi_rollout(struct OdgSim* sim, const float* mean_dev, float sigma, int
 int odg_mppi_reduce(const float* cost_dev, const float* actions_dev, int horizon, int n_samples, int act_dim,
                     float lambda, float* mean_out_dev, float* stats_dev, void* stream);
 
+/* ---- Batched MPPI: G robots planned in one launch each, each from its own start state (opendog_b200.mppi.BatchedMPPI).
+ * A samples handle of N = G * S environments holds G groups of S samples; sample n = g * S + s belongs to group g.
+ * Per plan: odg_mppi_broadcast -> odg_mppi_rollout_groups -> odg_mppi_reduce_groups, no host round trip.
+ *
+ * Copy robot `first_robot + g` of `robots` into samples [g S, (g + 1) S) for g in [0, groups), S = samples.n / groups,
+ * in one launch on the device (SoA to SoA): qpos, qvel, the solver's qacc warm start, step counter, gait index, gait
+ * matches, last action, desired velocity and `fresh` — every per-environment field the env-step reads. Invariant: when
+ * the two handles share model and config, a sample stepped with its robot's action reproduces that robot's step bit
+ * for bit (which is why the warm start is copied, not zeroed). ODG_ERR_INVALID, before any device work, for null
+ * handles, handles on different devices, different nq / nv / nu / task, groups < 1, first_robot < 0,
+ * first_robot + groups > robots.n, samples.n % groups != 0, or a samples handle created with auto_reset = 1. */
+int odg_mppi_broadcast(struct OdgSim* samples, const struct OdgSim* robots, int first_robot, int groups, void* stream);
+
+/* odg_mppi_rollout for `groups` groups of S = sim.n / groups samples: sample n = g * S + s follows the nominal
+ * sequence mean[g] and draws its noise exactly as a single-robot plan draws it for sample s with the 64-bit key
+ * seed + g. So group g equals odg_mppi_rollout(seed + g) on an S-sample handle holding the same start state (e.g.
+ * filled by odg_mppi_broadcast(first_robot = g, groups = 1)), bit for bit, action rows and costs; odg_mppi_rollout is
+ * the groups = 1 case. mean_dev [G][T][A]; actions_dev [T][N][A]; cost_dev [N]. ODG_ERR_INVALID when groups < 1 or
+ * sim.n % groups != 0, and for the arguments odg_mppi_rollout refuses. */
+int odg_mppi_rollout_groups(struct OdgSim* sim, int groups, const float* mean_dev, float sigma, int horizon, uint64_t seed,
+                            uint32_t iteration, const uint32_t* iteration_dev, float termination_cost, float* actions_dev,
+                            float* cost_dev, void* stream);
+
+/* odg_mppi_reduce per group: one 1024-thread block per group, the same fixed tree and in-order sample sums, so group g
+ * equals odg_mppi_reduce on a contiguous copy of actions[:, g S:(g + 1) S] bit for bit; odg_mppi_reduce is the
+ * groups = 1 case. actions_dev [T][G S][A]; cost_dev [G S]; mean_out_dev [G][T][A]; stats_dev [G][4] nullable, with
+ * stats[g][3] the argmin within group g. samples_per_group <= 12000. */
+int odg_mppi_reduce_groups(const float* cost_dev, const float* actions_dev, int horizon, int groups, int samples_per_group,
+                           int act_dim, float lambda, float* mean_out_dev, float* stats_dev, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -152,12 +152,16 @@ struct SimPtrs {            // SoA state in HBM: x[i*N + env]
 
 // MPPI mode of the step kernel (include/odg_mppi.h: odg_mppi_rollout): T > 0 turns one launch into a whole rollout —
 // every environment walks T env-steps, drawing its own action row before each one and accumulating its cost.
+// Environments form groups of S samples (odg_mppi_rollout_groups): sample g * S + s reads the nominal rows of group g and
+// draws the noise of sample s under the key seed + g.
 struct MppiArgs {
   int T;                          // horizon; 0 = ordinary step
+  int S;                          // samples per group (MPPI mode only)
+  int mean_stride;                // floats between the nominal sequences of consecutive groups
   float sigma, term_cost;
   uint32_t seed_lo, seed_hi, iteration;
   const uint32_t* iteration_dev;  // nullable: device-side plan counter (CUDA-graph replays draw fresh noise)
-  const float* mean;              // [T][A]
+  const float* mean;              // [G][T][A]
   float* actions;                 // [T][n][A]
   float* cost;                    // [n]
 };

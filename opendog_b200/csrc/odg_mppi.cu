@@ -29,15 +29,20 @@ __global__ void k_mppi_accum(const float* __restrict__ reward, const unsigned ch
 }
 
 constexpr int kRedThreads = 1024;
+// One block per group of S samples (block g reads samples [g S, (g + 1) S) of the [T][N][A] action tensor and writes
+// mean_out[g] and stats[g]); a group's arithmetic is that of a single-group call on a contiguous copy of its samples.
 __global__ void __launch_bounds__(kRedThreads) k_mppi_reduce(const float* __restrict__ cost, const float* __restrict__ actions, int T,
-                                                             int N, int A, float lambda, float* __restrict__ mean_out,
+                                                             int S, int N, int A, float lambda, float* __restrict__ mean_out,
                                                              float* __restrict__ stats) {
-  extern __shared__ float s_w[];                 // [N] weights
+  extern __shared__ float s_w[];                 // [S] weights
+  const int g = blockIdx.x;
+  cost += (size_t)g * S; actions += (size_t)g * S * A; mean_out += (size_t)g * T * A;
+  if (stats) stats += 4 * g;
   __shared__ float s_red[kRedThreads]; __shared__ int s_idx[kRedThreads];
   const int tid = threadIdx.x;
   // min cost (and its index), fixed tree
   float m = 3.4e38f; int mi = 0; float sum_c = 0.f;
-  for (int n = tid; n < N; n += kRedThreads) { const float c = cost[n]; sum_c += c; if (c < m) { m = c; mi = n; } }
+  for (int n = tid; n < S; n += kRedThreads) { const float c = cost[n]; sum_c += c; if (c < m) { m = c; mi = n; } }
   s_red[tid] = m; s_idx[tid] = mi;
   __syncthreads();
   for (int d = kRedThreads / 2; d > 0; d >>= 1) {
@@ -51,7 +56,7 @@ __global__ void __launch_bounds__(kRedThreads) k_mppi_reduce(const float* __rest
   __syncthreads();
   // weights and their sum
   float ws = 0.f;
-  for (int n = tid; n < N; n += kRedThreads) { const float w = expf(-(cost[n] - cmin) / lambda); s_w[n] = w; ws += w; }
+  for (int n = tid; n < S; n += kRedThreads) { const float w = expf(-(cost[n] - cmin) / lambda); s_w[n] = w; ws += w; }
   s_red[tid] = ws;
   __syncthreads();
   for (int d = kRedThreads / 2; d > 0; d >>= 1) { if (tid < d) s_red[tid] += s_red[tid + d]; __syncthreads(); }
@@ -60,13 +65,13 @@ __global__ void __launch_bounds__(kRedThreads) k_mppi_reduce(const float* __rest
   s_red[tid] = sum_c;
   __syncthreads();
   for (int d = kRedThreads / 2; d > 0; d >>= 1) { if (tid < d) s_red[tid] += s_red[tid + d]; __syncthreads(); }
-  if (tid == 0 && stats) { stats[0] = cmin; stats[1] = s_red[0] / (float)N; stats[2] = wsum; stats[3] = (float)imin; }
+  if (tid == 0 && stats) { stats[0] = cmin; stats[1] = s_red[0] / (float)S; stats[2] = wsum; stats[3] = (float)imin; }
   // weighted mean per (t, a): thread per output element, samples summed in index order
   for (int o = tid; o < T * A; o += kRedThreads) {
     const int t = o / A, a = o % A;
     const float* p = actions + (size_t)t * N * A + a;
     float acc = 0.f;
-    for (int n = 0; n < N; n++) acc += s_w[n] * p[(size_t)n * A];
+    for (int n = 0; n < S; n++) acc += s_w[n] * p[(size_t)n * A];
     mean_out[o] = acc / wsum;
   }
 }
@@ -98,11 +103,20 @@ int odg_mppi_reduce(const float* cost_dev, const float* actions_dev, int horizon
                     float* mean_out_dev, float* stats_dev, void* stream) {
   if (!cost_dev || !actions_dev || !mean_out_dev || horizon < 1 || n_samples < 1 || n_samples > 12000 || act_dim < 1 || !(lambda > 0.f))
     return set_error(ODG_ERR_INVALID, "odg_mppi_reduce: bad arguments (n_samples <= 12000)");
-  // [n_samples] weights in dynamic shared memory next to 8 KB of static reduction rows: above 48 KB in total the kernel
-  // needs the opt-in limit (n_samples > ~10000)
-  CUDA_TRY(cudaFuncSetAttribute(k_mppi_reduce, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)((size_t)n_samples * sizeof(float))));
-  k_mppi_reduce<<<1, kRedThreads, (size_t)n_samples * sizeof(float), static_cast<cudaStream_t>(stream)>>>(
-      cost_dev, actions_dev, horizon, n_samples, act_dim, lambda, mean_out_dev, stats_dev);
+  return odg_mppi_reduce_groups(cost_dev, actions_dev, horizon, 1, n_samples, act_dim, lambda, mean_out_dev, stats_dev, stream);
+}
+
+int odg_mppi_reduce_groups(const float* cost_dev, const float* actions_dev, int horizon, int groups, int samples_per_group,
+                           int act_dim, float lambda, float* mean_out_dev, float* stats_dev, void* stream) {
+  if (!cost_dev || !actions_dev || !mean_out_dev || horizon < 1 || groups < 1 || samples_per_group < 1 ||
+      samples_per_group > 12000 || act_dim < 1 || !(lambda > 0.f) || (long long)groups * samples_per_group > 0x7fffffff)
+    return set_error(ODG_ERR_INVALID, "odg_mppi_reduce_groups: bad arguments (samples_per_group <= 12000)");
+  // [S] weights in dynamic shared memory next to 8 KB of static reduction rows: above 48 KB in total the kernel
+  // needs the opt-in limit (S > ~10000)
+  const size_t smem = (size_t)samples_per_group * sizeof(float);
+  CUDA_TRY(cudaFuncSetAttribute(k_mppi_reduce, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k_mppi_reduce<<<groups, kRedThreads, smem, static_cast<cudaStream_t>(stream)>>>(
+      cost_dev, actions_dev, horizon, samples_per_group, groups * samples_per_group, act_dim, lambda, mean_out_dev, stats_dev);
   CUDA_TRY(cudaGetLastError());
   return ODG_OK;
 }

@@ -70,14 +70,20 @@ __global__ void __launch_bounds__(ODG_MAX_BLOCK, ODG_MIN_BLOCKS) k_step(const __
   for (int base = blockIdx.x * envs_per_block; base < P.N; base += gridDim.x * envs_per_block) {
     const int env = base + (threadIdx.x >> 5) * envs_per_warp + (lane >> 2);
     if (env >= P.N) continue;
+    // MPPI groups, once per sample: env = g * S + s. Padding environments (env >= n) take the last group, so no mean
+    // pointer goes past it; they draw no rows.
+    const int g = M.T > 0 ? min(env, P.n - 1) / M.S : 0, s = env - g * M.S;
     float cost = 0.f;
     bool alive = true;
     for (int t = 0; t < horizon; t++) {
       const float* action = A.action;
       if (M.T > 0) {
         float* row = M.actions + (size_t)t * P.n * C.nu;
-        if (leg == 0 && env < P.n)
-          odg::mppi_sample_row(M.mean + (size_t)t * C.nu, M.sigma, env, C.nu, M.seed_lo, M.seed_hi, iteration, (uint32_t)t, row);
+        if (leg == 0 && env < P.n) {
+          const uint64_t key = ((((uint64_t)M.seed_hi) << 32) | M.seed_lo) + (uint64_t)g;
+          odg::mppi_sample_row(M.mean + (size_t)g * M.mean_stride + (size_t)t * C.nu, M.sigma, s, C.nu, (uint32_t)key,
+                               (uint32_t)(key >> 32), iteration, (uint32_t)t, row + (size_t)(env - s) * C.nu);
+        }
         __syncwarp(gm);                            // the group's other lanes read the row lane 0 just wrote
         action = row;
       }
@@ -126,6 +132,21 @@ template <typename T>
 __global__ void k_copy(T* dst, const T* src, long long n) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) dst[i] = src[i];
+}
+
+// odg_mppi_broadcast: sample n of D <- robot first + n / S of R, every per-environment field env_step reads (SoA to SoA)
+__global__ void k_mppi_broadcast(const SimPtrs D, const SimPtrs R, int first, int S, int nq, int nv, int nu) {
+  const int n = blockIdx.x * blockDim.x + threadIdx.x;
+  if (n >= D.n) return;
+  const int r = first + n / S;
+  for (int k = 0; k < nq; k++) D.qpos[(size_t)k * D.N + n] = R.qpos[(size_t)k * R.N + r];
+  for (int k = 0; k < nv; k++) {
+    D.qvel[(size_t)k * D.N + n] = R.qvel[(size_t)k * R.N + r];
+    D.warm[(size_t)k * D.N + n] = R.warm[(size_t)k * R.N + r];
+  }
+  for (int k = 0; k < nu; k++) D.last_action[(size_t)k * D.N + n] = R.last_action[(size_t)k * R.N + r];
+  for (int k = 0; k < 3; k++) D.desvel[(size_t)k * D.N + n] = R.desvel[(size_t)k * R.N + r];
+  D.step[n] = R.step[r]; D.gait_idx[n] = R.gait_idx[r]; D.gait_cnt[n] = R.gait_cnt[r]; D.fresh[n] = R.fresh[r];
 }
 
 }  // namespace
@@ -229,6 +250,32 @@ struct DeviceGuard {
   explicit DeviceGuard(int dev) { cudaGetDevice(&prev); if (prev != dev) cudaSetDevice(dev); else prev = -1; }
   ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
 };
+
+// odg_mppi_rollout (groups = 1) and odg_mppi_rollout_groups: one launch of the step kernel in MPPI mode
+int mppi_rollout(OdgSim* s, int groups, const float* mean_dev, float sigma, int horizon, uint64_t seed, uint32_t iteration,
+                 const uint32_t* iteration_dev, float termination_cost, float* actions_dev, float* cost_dev, cudaStream_t st,
+                 const char* who) {
+  if (!s || !mean_dev || !actions_dev || !cost_dev || horizon < 1 || !(sigma >= 0.f) || groups < 1)
+    return fail(ODG_ERR_INVALID, std::string(who) + ": bad arguments");
+  if (s->P.n % groups) return fail(ODG_ERR_INVALID, std::string(who) + ": the handle's environments are not a whole number of groups");
+  if (s->prep.C.auto_reset) return fail(ODG_ERR_INVALID, std::string(who) + ": the handle must be created with auto_reset = 0");
+  DeviceGuard guard(s->device);
+  DevConst C = s->prep.C;
+  C.lockstep = 0;                                  // samples leave the horizon loop at different times: no block barriers
+  odg::MppiArgs M;
+  M.T = horizon; M.S = s->P.n / groups; M.mean_stride = horizon * C.nu; M.sigma = sigma; M.term_cost = termination_cost;
+  M.seed_lo = (uint32_t)seed; M.seed_hi = (uint32_t)(seed >> 32); M.iteration = iteration; M.iteration_dev = iteration_dev;
+  M.mean = mean_dev; M.actions = actions_dev; M.cost = cost_dev;
+  StepArgs A;
+  fill_args(&A, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0);
+  // every sample gets its own 4-lane group for the whole horizon: one tile per block, never a second wave
+  const int epb = (s->step_block / 32) * (s->step_lanes / 4);
+  const int grid = (s->P.N + epb - 1) / epb;
+  step_kernel_fn(C, s->step_fat != 0)<<<grid, s->step_block, s->smem_step, st>>>(C, s->P, A, M, s->d_lc, s->d_gc, s->d_vert, s->L, s->step_lanes);
+  s->launches++;
+  CUDA_TRY(cudaGetLastError());
+  return ODG_OK;
+}
 
 }  // namespace
 
@@ -365,23 +412,31 @@ int odg_step_host(OdgSim* s, const float* action_host, float* action_pinned, flo
 
 int odg_mppi_rollout(OdgSim* s, const float* mean_dev, float sigma, int horizon, uint64_t seed, uint32_t iteration,
                      const uint32_t* iteration_dev, float termination_cost, float* actions_dev, float* cost_dev, void* stream) {
-  if (!s || !mean_dev || !actions_dev || !cost_dev || horizon < 1 || !(sigma >= 0.f))
-    return fail(ODG_ERR_INVALID, "odg_mppi_rollout: bad arguments");
-  if (s->prep.C.auto_reset) return fail(ODG_ERR_INVALID, "odg_mppi_rollout: the handle must be created with auto_reset = 0");
-  DeviceGuard guard(s->device);
-  DevConst C = s->prep.C;
-  C.lockstep = 0;                                  // samples leave the horizon loop at different times: no block barriers
-  odg::MppiArgs M;
-  M.T = horizon; M.sigma = sigma; M.term_cost = termination_cost;
-  M.seed_lo = (uint32_t)seed; M.seed_hi = (uint32_t)(seed >> 32); M.iteration = iteration; M.iteration_dev = iteration_dev;
-  M.mean = mean_dev; M.actions = actions_dev; M.cost = cost_dev;
-  StepArgs A;
-  fill_args(&A, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0);
-  // every sample gets its own 4-lane group for the whole horizon: one tile per block, never a second wave
-  const int epb = (s->step_block / 32) * (s->step_lanes / 4);
-  const int grid = (s->P.N + epb - 1) / epb;
-  step_kernel_fn(C, s->step_fat != 0)<<<grid, s->step_block, s->smem_step, static_cast<cudaStream_t>(stream)>>>(C, s->P, A, M, s->d_lc, s->d_gc, s->d_vert, s->L, s->step_lanes);
-  s->launches++;
+  return mppi_rollout(s, 1, mean_dev, sigma, horizon, seed, iteration, iteration_dev, termination_cost, actions_dev, cost_dev,
+                      static_cast<cudaStream_t>(stream), "odg_mppi_rollout");
+}
+
+int odg_mppi_rollout_groups(OdgSim* s, int groups, const float* mean_dev, float sigma, int horizon, uint64_t seed,
+                            uint32_t iteration, const uint32_t* iteration_dev, float termination_cost, float* actions_dev,
+                            float* cost_dev, void* stream) {
+  return mppi_rollout(s, groups, mean_dev, sigma, horizon, seed, iteration, iteration_dev, termination_cost, actions_dev,
+                      cost_dev, static_cast<cudaStream_t>(stream), "odg_mppi_rollout_groups");
+}
+
+int odg_mppi_broadcast(OdgSim* samples, const OdgSim* robots, int first_robot, int groups, void* stream) {
+  if (!samples || !robots) return fail(ODG_ERR_INVALID, "odg_mppi_broadcast: null handle");
+  const DevConst& D = samples->prep.C; const DevConst& R = robots->prep.C;
+  if (samples->device != robots->device) return fail(ODG_ERR_INVALID, "odg_mppi_broadcast: the handles are on different devices");
+  if (D.nq != R.nq || D.nv != R.nv || D.nu != R.nu || D.task != R.task)
+    return fail(ODG_ERR_INVALID, "odg_mppi_broadcast: the handles differ in nq / nv / nu / task");
+  if (groups < 1 || first_robot < 0 || first_robot > robots->P.n - groups)
+    return fail(ODG_ERR_INVALID, "odg_mppi_broadcast: robots [first_robot, first_robot + groups) out of range");
+  if (samples->P.n % groups) return fail(ODG_ERR_INVALID, "odg_mppi_broadcast: the samples are not a whole number of groups");
+  if (D.auto_reset) return fail(ODG_ERR_INVALID, "odg_mppi_broadcast: the samples handle must be created with auto_reset = 0");
+  DeviceGuard guard(samples->device);
+  k_mppi_broadcast<<<(samples->P.n + 127) / 128, 128, 0, static_cast<cudaStream_t>(stream)>>>(
+      samples->P, robots->P, first_robot, samples->P.n / groups, D.nq, D.nv, D.nu);
+  samples->launches++;
   CUDA_TRY(cudaGetLastError());
   return ODG_OK;
 }

@@ -63,6 +63,7 @@ class BatchedWalkEnv:
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         if self.device.index is None:
             self.device = torch.device("cuda", torch.cuda.current_device())
+        self.model = model
         self.desc = load_compiled(model)
         self._model = to_struct(self.desc)
         self.cfg = _lib.OdgEnvConfig()

@@ -31,6 +31,7 @@ SYMBOLS = [
     "odg_terrain_data",
     # MPPI (include/odg_mppi.h)
     "odg_mppi_sample", "odg_mppi_accumulate", "odg_mppi_reduce", "odg_mppi_rollout",
+    "odg_mppi_broadcast", "odg_mppi_rollout_groups", "odg_mppi_reduce_groups",
 ]
 
 
@@ -136,6 +137,10 @@ def load():
     L.odg_mppi_accumulate.argtypes = [_vp, _vp, C.c_int, C.c_float, _vp, _vp, _vp]
     L.odg_mppi_rollout.argtypes = [_vp, _vp, C.c_float, C.c_int, C.c_uint64, C.c_uint32, _vp, C.c_float, _vp, _vp, _vp]
     L.odg_mppi_reduce.argtypes = [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_float, _vp, _vp, _vp]
+    L.odg_mppi_broadcast.argtypes = [_vp, _vp, C.c_int, C.c_int, _vp]
+    L.odg_mppi_rollout_groups.argtypes = [_vp, C.c_int, _vp, C.c_float, C.c_int, C.c_uint64, C.c_uint32, _vp, C.c_float, _vp, _vp,
+                                          _vp]
+    L.odg_mppi_reduce_groups.argtypes = [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, _vp, _vp, _vp]
     L.odg_last_error.restype = C.c_char_p
     L.odg_version.restype = C.c_char_p
     _lib = L
