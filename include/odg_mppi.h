@@ -42,7 +42,12 @@ int odg_mppi_rollout(struct OdgSim* sim, const float* mean_dev, float sigma, int
 
 /* Information-theoretic MPPI update, one block, fixed summation order (deterministic):
  *   w[n] = exp(-(cost[n] - min cost) / lambda);  mean_out[t][a] = sum_n w[n] action[t][n][a] / sum_n w[n]
- * actions_dev [T][N][A]; mean_out_dev [T][A]; stats_dev [4] f32 = (min cost, mean cost, sum w, argmin) nullable. */
+ * actions_dev [T][N][A]; mean_out_dev [T][A]; stats_dev [4] f32 = (min cost, mean cost, sum w, argmin) nullable.
+ * Non-finite costs (a sample whose rollout state went NaN or infinite): only samples with a finite cost take part in
+ * the min, the argmin, the mean cost and the weights; a non-finite cost gets weight exactly 0, so the result is that of
+ * the same costs with it replaced by any finite value whose weight underflows to 0. If no cost is finite, mean_out = 0
+ * and stats = (+inf, NaN, 0, -1). With every cost finite the arithmetic is the plain formula above.
+ * (tests/test_gpu_mppi_numerics.py) */
 int odg_mppi_reduce(const float* cost_dev, const float* actions_dev, int horizon, int n_samples, int act_dim,
                     float lambda, float* mean_out_dev, float* stats_dev, void* stream);
 
@@ -72,7 +77,9 @@ int odg_mppi_rollout_groups(struct OdgSim* sim, int groups, const float* mean_de
 /* odg_mppi_reduce per group: one 1024-thread block per group, the same fixed tree and in-order sample sums, so group g
  * equals odg_mppi_reduce on a contiguous copy of actions[:, g S:(g + 1) S] bit for bit; odg_mppi_reduce is the
  * groups = 1 case. actions_dev [T][G S][A]; cost_dev [G S]; mean_out_dev [G][T][A]; stats_dev [G][4] nullable, with
- * stats[g][3] the argmin within group g. samples_per_group <= 12000. */
+ * stats[g][3] the argmin within group g. samples_per_group <= 12000. Non-finite costs as in odg_mppi_reduce, per group:
+ * a group with no finite cost writes mean_out[g] = 0 (the nominal an ended episode restarts from) and
+ * stats[g] = (+inf, NaN, 0, -1); the other groups are unaffected. */
 int odg_mppi_reduce_groups(const float* cost_dev, const float* actions_dev, int horizon, int groups, int samples_per_group,
                            int act_dim, float lambda, float* mean_out_dev, float* stats_dev, void* stream);
 

@@ -31,6 +31,8 @@ __global__ void k_mppi_accum(const float* __restrict__ reward, const unsigned ch
 constexpr int kRedThreads = 1024;
 // One block per group of S samples (block g reads samples [g S, (g + 1) S) of the [T][N][A] action tensor and writes
 // mean_out[g] and stats[g]); a group's arithmetic is that of a single-group call on a contiguous copy of its samples.
+// Only samples with a finite cost take part: a NaN or infinite cost (a rollout whose state went non-finite) is left out
+// of the min, the argmin and the cost sum and gets weight exactly 0. A group with no finite cost writes a zero mean.
 __global__ void __launch_bounds__(kRedThreads) k_mppi_reduce(const float* __restrict__ cost, const float* __restrict__ actions, int T,
                                                              int S, int N, int A, float lambda, float* __restrict__ mean_out,
                                                              float* __restrict__ stats) {
@@ -40,9 +42,12 @@ __global__ void __launch_bounds__(kRedThreads) k_mppi_reduce(const float* __rest
   if (stats) stats += 4 * g;
   __shared__ float s_red[kRedThreads]; __shared__ int s_idx[kRedThreads];
   const int tid = threadIdx.x;
-  // min cost (and its index), fixed tree
-  float m = 3.4e38f; int mi = 0; float sum_c = 0.f;
-  for (int n = tid; n < S; n += kRedThreads) { const float c = cost[n]; sum_c += c; if (c < m) { m = c; mi = n; } }
+  // min finite cost (and its index; -1 if none), fixed tree
+  float m = INFINITY; int mi = -1; float sum_c = 0.f; int nfin = 0;
+  for (int n = tid; n < S; n += kRedThreads) {
+    const float c = cost[n];
+    if (isfinite(c)) { sum_c += c; nfin++; if (c < m) { m = c; mi = n; } }
+  }
   s_red[tid] = m; s_idx[tid] = mi;
   __syncthreads();
   for (int d = kRedThreads / 2; d > 0; d >>= 1) {
@@ -54,25 +59,33 @@ __global__ void __launch_bounds__(kRedThreads) k_mppi_reduce(const float* __rest
   }
   const float cmin = s_red[0]; const int imin = s_idx[0];
   __syncthreads();
-  // weights and their sum
+  // weights and their sum (with the count of finite costs, summed in the same tree)
   float ws = 0.f;
-  for (int n = tid; n < S; n += kRedThreads) { const float w = expf(-(cost[n] - cmin) / lambda); s_w[n] = w; ws += w; }
-  s_red[tid] = ws;
+  for (int n = tid; n < S; n += kRedThreads) {
+    const float c = cost[n];
+    const float w = isfinite(c) ? expf(-(c - cmin) / lambda) : 0.f;
+    s_w[n] = w; ws += w;
+  }
+  s_red[tid] = ws; s_idx[tid] = nfin;
   __syncthreads();
-  for (int d = kRedThreads / 2; d > 0; d >>= 1) { if (tid < d) s_red[tid] += s_red[tid + d]; __syncthreads(); }
-  const float wsum = s_red[0];
+  for (int d = kRedThreads / 2; d > 0; d >>= 1) {
+    if (tid < d) { s_red[tid] += s_red[tid + d]; s_idx[tid] += s_idx[tid + d]; }
+    __syncthreads();
+  }
+  const float wsum = s_red[0]; const int nfin_all = s_idx[0];
   __syncthreads();
   s_red[tid] = sum_c;
   __syncthreads();
   for (int d = kRedThreads / 2; d > 0; d >>= 1) { if (tid < d) s_red[tid] += s_red[tid + d]; __syncthreads(); }
-  if (tid == 0 && stats) { stats[0] = cmin; stats[1] = s_red[0] / (float)S; stats[2] = wsum; stats[3] = (float)imin; }
+  // no finite cost: (+inf, 0 / 0 = NaN, 0, -1)
+  if (tid == 0 && stats) { stats[0] = cmin; stats[1] = s_red[0] / (float)nfin_all; stats[2] = wsum; stats[3] = (float)imin; }
   // weighted mean per (t, a): thread per output element, samples summed in index order
   for (int o = tid; o < T * A; o += kRedThreads) {
     const int t = o / A, a = o % A;
     const float* p = actions + (size_t)t * N * A + a;
     float acc = 0.f;
     for (int n = 0; n < S; n++) acc += s_w[n] * p[(size_t)n * A];
-    mean_out[o] = acc / wsum;
+    mean_out[o] = imin < 0 ? 0.f : acc / wsum;
   }
 }
 }  // namespace
